@@ -7,6 +7,7 @@ points, 256-d features, 1024 CAD samples.  Under torchrun every rank runs the sa
 sharded, no data-path collective) and the step ends with the one all-gather of final poses.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          our arm
+  python bench.py ... --dump-outputs DIR                        our arm, and the poses of its last timed step as DIR/*.npy
   python bench.py --impl reference ...                          the reference algorithm on the host cores (oracle port)
 """
 import argparse
@@ -20,6 +21,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 WORKLOAD = "pem_matching_32x2048x2048"
@@ -27,6 +29,7 @@ B_PER_GPU, N_PTS, N_MODEL, C_FEAT = 32, 2048, 1024, 256
 METRIC, UNIT = "poses/sec", "poses/s"
 REF_ARM_B = 1
 CPU_SAMPLE_B = 8
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def peaks():
@@ -113,6 +116,20 @@ def host_threads() -> int:
         except (OSError, ValueError, IndexError):
             continue
     return max(1, n)
+
+
+def dump_outputs(out_dir: str, arrays: dict, limit_bytes: int = DUMP_LIMIT_BYTES):
+    """write every array as out_dir/<name>.npy in float32.  Above limit_bytes in all, the same fixed, seeded sample of
+    proposals (rows along the first axis, kept in order) is written for every array."""
+    arrays = {k: v.detach().to(torch.float32).cpu() for k, v in arrays.items()}
+    rows = next(iter(arrays.values())).shape[0]
+    per_row = sum(v[0].numel() * 4 for v in arrays.values()) if rows else 0
+    if rows * per_row > limit_bytes:
+        keep = torch.randperm(rows, generator=torch.Generator().manual_seed(0))[:limit_bytes // per_row].sort()[0]
+        arrays = {k: v[keep] for k, v in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.numpy())
 
 
 def cpu_oracle_throughput(reps: int, threads: int, nprop: int = 0):
@@ -414,7 +431,13 @@ def main():
     ap.add_argument("--workload", default="pem", choices=["pem", "ism", "ycbv", "lmo"],
                     help="pem: BASELINE config #2 (headline); ism: config #3, SAM ViT-H encoder + template scoring; ycbv / lmo: "
                          "configs #5 / #4, strong scaling of one fixed frame set over the ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the poses Net.forward returned in the last one (rank 0: init_R, init_t, "
+                         "pred_R, pred_t, pred_pose_score) as DIR/<name>.npy, float32; the inputs are seeded, so two builds "
+                         "compare output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "pem"):
+        ap.error("--dump-outputs writes the outputs of the pem workload of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload == "ism":
@@ -425,6 +448,7 @@ def main():
     import torch.distributed as dist
     from sam6d_b200 import synth                  # seeded weights + synthetic inputs (no oracle code on this arm)
     from sam6d_b200 import _lib, dist as sdist
+    from sam6d_b200.graph import OUT_KEYS
     from sam6d_b200.pem import Net
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -465,10 +489,13 @@ def main():
     h2d_bytes = sum(v.numel() * v.element_size() for v in host[0].values())
     gen = torch.Generator(device=dev).manual_seed(1 + rank)
 
+    last = {}
+
     def step_resident(i):
         ep = dict(resident[i % 2])
         rand = torch.rand(B, synth.N_PROPOSAL1 * 3, device=dev, generator=gen)
         out = net(ep, rand=rand)
+        last["out"] = out
         poses = sdist.pack_poses(out)
         return sdist.all_gather_poses(poses)
 
@@ -553,6 +580,8 @@ def main():
     if sampler:
         sampler.start()
     ms, launches, _ = timed(step_resident, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {k: last["out"][k] for k, _ in OUT_KEYS})
     # dominant-kernel roofline: same steps again with CUDA events around every launch of the kernels the roofline report names
     # (the stream over E; the attention kernel that consumes its scores; the geometric-embedding kernel that writes E)
     from sam6d_b200 import pem as _pem

@@ -2,8 +2,9 @@
 
 Compiles the REFERENCE's own PointNet++ CUDA extension (pointnet2._ext) from the sources where they lie under
 /root/reference, into oracle/_ref/ (git-ignored; travels to the GPU box with the snapshot).  No reference source is copied
-into this repository.  tests/test_gpu_pn2_ref.py loads the resulting module on the GPU box and uses it to pin both the C
-restatement (oracle/pn2_oracle.c) and the sam6d_b200 kernels against the reference kernels' actual outputs.
+into this repository.  tools/make_golden_pn2_ref.py runs the resulting module on a GPU and stores the reference kernels'
+outputs as tests/golden/pn2_ref.pt, against which tests/test_gpu_pn2_ref.py pins both the C restatement (oracle/pn2_oracle.c)
+and the sam6d_b200 kernels; bench.py times it next to ours when it is present.
 
 The reference's setup.py does not build as shipped (relative include_dirs, PEM/model/pointnet2/setup.py:23), so this is our
 own recipe: torch.utils.cpp_extension.load with an absolute include path and an sm_100 target.

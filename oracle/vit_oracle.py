@@ -6,8 +6,8 @@ CPU restatement (torch fp32) of the PEM RGB branch, PEM/model/feature_extraction
     get_img_feats       ViTEncoder.get_img_feats :166-167 = get_chosen_pixel_feats (PEM/utils/model_utils.py:69-81)
 Parity status:
   * everything below the ViT trunk (concatenation of the 4 pyramid levels, output_upscaling, the reshape / permute to the
-    56 x 56 map, F.interpolate(bilinear, align_corners=False), the pixel gather) follows reference code that is present in
-    /root/reference and is checked against model_utils.get_chosen_pixel_feats by tests/test_oracle_vit.py;
+    56 x 56 map, F.interpolate(bilinear, align_corners=False), the pixel gather) follows reference code, and the gather is
+    checked against the output of model_utils.get_chosen_pixel_feats (tests/golden/vit_gather.pt) by tests/test_oracle_vit.py;
   * the trunk itself is timm's VisionTransformer, which the reference neither vendors nor pins (PEM/dependencies.sh:4,
     environment.yaml:34) and which is absent here: PARITY UNPINNED.  The restatement follows timm >= 0.6 semantics:
     patch_embed = Conv2d(3, D, 16, 16) -> flatten(2).transpose(1,2); _pos_embed = cat(cls_token, x) + pos_embed;

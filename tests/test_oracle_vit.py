@@ -1,34 +1,24 @@
-"""CPU: the part of oracle/vit_oracle.py that restates reference code present in /root/reference (pixel gather) is checked
-against that code when the reference tree is available; the bilinear-gather formula used by the CUDA kernel is checked against
-F.interpolate on random maps.  (The timm trunk is unpinned, see the oracle header.)"""
+"""CPU: the part of oracle/vit_oracle.py that restates reference code (pixel gather) is checked against that code's output
+(tests/golden/vit_gather.pt, tools/make_golden_vit_gather.py); the bilinear-gather formula used by the CUDA kernel is checked
+against F.interpolate on random maps.  (The timm trunk is unpinned, see the oracle header.)"""
 import os
-import sys
 
-import pytest
 import torch
 import torch.nn.functional as F
 
 from oracle import vit_oracle as vo
 
-REF_UTILS = "/root/reference/SAM-6D/Pose_Estimation_Model/utils"
 
-
-def test_chosen_pixel_feats_matches_reference_function():
-    if not os.path.isdir(REF_UTILS):
-        pytest.skip("reference tree not present (GPU box)")
-    import builtins
-    builtins.__POINTNET2_SETUP__ = True
-    for p in (REF_UTILS, os.path.join(os.path.dirname(REF_UTILS), "model", "pointnet2")):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    try:
-        import model_utils as mu                                  # reference module, read only
-    except Exception as e:                                        # optional dependency of the reference missing
-        pytest.skip(f"reference model_utils not importable: {e}")
+def gather_inputs():
     g = torch.Generator().manual_seed(0)
     img = torch.randn(2, 16, 20, 24, generator=g)
     choose = torch.randint(0, 20 * 24, (2, 50), generator=g)
-    assert torch.equal(vo.chosen_pixel_feats(img, choose), mu.get_chosen_pixel_feats(img, choose))
+    return img, choose
+
+
+def test_chosen_pixel_feats_matches_reference_function(golden_dir):
+    want = torch.load(os.path.join(golden_dir, "vit_gather.pt"), weights_only=False)["feats"]
+    assert torch.equal(vo.chosen_pixel_feats(*gather_inputs()), want)
 
 
 def test_bilinear_gather_formula_matches_interpolate():
